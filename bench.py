@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Point-SAM hot path (BASELINE.json metric: point-clouds/sec, N=32768, ViT-L, 512x64 groups).
 
-  python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--config c2] [--no-graph]
+  python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--config c2] [--no-graph] [--dump-outputs DIR]
 
 Headline workload (config c2, BASELINE.json configs[1]): independent single-cloud requests (B=1, N=32768, G=512, K=64,
 EVA02-L, one point prompt) through FPS + kNN grouping + mini-PointNet + ViT-L encoder + prompt decoder -> mask logits.
@@ -12,6 +12,15 @@ driver's short `--steps 20` run still times >= 0.5 s; `value` stays clouds/s.
   e2e   : the same through the public predictor API with HOST (pinned) buffers: H2D of cloud + prompts and D2H of
           logits + IoU inside the timed region, every result read on the host.
 Multi-GPU: one process per GPU (torchrun), clouds sharded by rank, weights replicated.
+
+`--dump-outputs DIR` writes what the last timed step of the `value` arm returned: `masks.npy` (mask logits of every
+request of the step, [clouds, masks, N]) and `iou.npy` ([clouds, masks]), float32, plus `c3_iou_rows.npy` (per-cloud IoU
+of every prompt iteration) when the c3 arm runs; a rank > 0 adds `_rank<r>` to the names.  All files of all ranks stay
+within 64 MB: past that, the logits keep a fixed, seeded sample of the N points.  Only the repo arm dumps.  A lane's
+outputs are overwritten by its next request within the step, so the last timed step also copies each request's logits
+and IoU on the lane's stream: the `value` of a dump run includes those 2 x requests device-to-device copies.  The
+inputs depend only on the arguments, so two builds can be compared output for output.  Compare them with a tolerance,
+because repeated runs of one build agree only to rounding: split-K GEMMs accumulate with atomics.
 
 The same line carries "c3" (BASELINE.json configs[2], run after the c2 arms unless --no-c3): a FIXED batch of 32 clouds
 sharded contiguously over the ranks (strong scaling), 3 prompt iterations of the evaluation loop
@@ -33,6 +42,7 @@ import threading
 import time
 
 REPO = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # a benchmark run writes nothing into the tree (it may be read-only)
 for p in (REPO, os.path.join(REPO, "point-sam_b200")):
     if p not in sys.path:
         sys.path.insert(0, p)
@@ -53,6 +63,28 @@ CONFIGS = {
 C3 = {"c3": ("eva02_large_patch14_448", 32768, 512, 64, 32, 4, 3, 1),
       "c3tiny": ("eva02_test_tiny", 2048, 64, 16, 32, 4, 3, 1)}
 METRIC = "point-clouds/sec (N=32768, ViT-L, 512x64 groups)"  # BASELINE.json metric; other --config values are side runs
+
+
+DUMP_BYTES = 64 << 20  # --dump-outputs: cap on the bytes written by all ranks together
+
+
+def write_outputs(out_dir, arrays, budget, n_points=0, tag=""):
+    """Write every array as out_dir/<name><tag>.npy in float32, in at most `budget` bytes.  Past the budget, the arrays
+    whose last axis holds the n_points points of a cloud keep a fixed, seeded sample of those points, so runs with the
+    same arguments stay comparable element for element."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: a.detach().float().cpu() for k, a in arrays.items()}
+    budget -= 1024 * len(arrays)  # .npy headers
+    total = sum(a.numel() * 4 for a in arrays.values())
+    if n_points and total > budget:
+        per_point = sum(a[..., 0].numel() * 4 for a in arrays.values() if a.shape[-1] == n_points)
+        keep = max(1, (budget - (total - per_point * n_points)) // per_point)
+        idx = torch.randperm(n_points, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        arrays = {k: a[..., idx] if a.shape[-1] == n_points else a for k, a in arrays.items()}
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}{tag}.npy"), a.numpy())
 
 
 def peaks():
@@ -145,14 +177,13 @@ def cpu_reference_throughput(cfg, steps: int, warmup: int):
 
 
 def run_reference(args):
-    """One JSON line; a bounded sample (requests of the workload, timed one by one on the host cores)."""
+    """One JSON line: --steps requests of the workload after --warmup untimed ones, timed one by one on the host cores."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
     name = args.config if args.config in CONFIGS else "c2"
     cfg = CONFIGS[name]
-    steps = max(1, min(args.steps, 20))
-    warm = max(1, min(args.warmup, 3))
+    steps, warm = args.steps, args.warmup
     v, ms, cores = cpu_reference_throughput(cfg, steps, warm)
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "clouds/s", "n_gpus": args.gpus, "steps": steps,
             "warmup": warm, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -173,7 +204,7 @@ def run_gpu_reference(args):
     from pc_sam.model import build_point_sam
 
     enc, N, G, K, bpg, P, kind = CONFIGS[args.config]
-    steps, warmup = max(1, min(args.steps, 10)), max(1, min(args.warmup, 3))
+    steps, warmup = args.steps, args.warmup
     dev = torch.device("cuda", 0)
     torch.cuda.set_device(dev)
     ref = build_ref.load_ref()
@@ -339,7 +370,7 @@ def only_regime(pp, keep, reps: int):
 # --------------------------------------------------------------------------------------------------
 # config c3: fixed batch sharded over the ranks, evaluation loop, all_gather of the IoU rows inside the timed region
 # --------------------------------------------------------------------------------------------------
-def run_c3(name, args, model, dev, dist, rank, world, barrier):
+def run_c3(name, args, model, dev, dist, rank, world, barrier, outputs=None):
     from pc_sam.model.loss import compute_iou
     from psam_b200 import synth
     from psam_b200.parallel import gather_metric, plan_graph_chunks, shard_range
@@ -414,6 +445,8 @@ def run_c3(name, args, model, dev, dist, rank, world, barrier):
     steps = max(1, args.steps)
     timed(devin, False, max(3, min(args.warmup, 5)))
     ms_dev = timed(devin, False, steps)
+    if outputs is not None:  # this rank's per-cloud IoU rows of the last timed step
+        outputs[f"{name}_iou_rows"] = rows.clone()
     timed(host, True, 3)
     ms_e2e = timed(host, True, steps)
     for ln in lanes:
@@ -450,7 +483,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-reference", action="store_true", help="skip the same-GPU PyTorch-eager reference timing")
     ap.add_argument("--no-roofline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy "
+                    "(repo arm only; its copies run inside that step)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the repo arm (--impl ours) only")
     if args.impl == "reference":
         return run_reference(args)
     if args.impl == "gpu-reference":
@@ -460,6 +501,7 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    dump_tag = f"_rank{rank}" if rank else ""
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     dist = None
@@ -485,7 +527,10 @@ def main():
         sampler = ClockSampler(local)
         if rank == 0:
             sampler.start()
-        r = run_c3(args.config, args, model, dev, dist, rank, world, barrier)
+        outputs = {} if args.dump_outputs else None
+        r = run_c3(args.config, args, model, dev, dist, rank, world, barrier, outputs)
+        if outputs:
+            write_outputs(args.dump_outputs, outputs, DUMP_BYTES // world, tag=dump_tag)
         if rank == 0:
             r.update({"metric": "point-clouds/sec (fixed batch of 32 clouds sharded over the ranks, 3 prompt iterations)",
                       "warmup": args.warmup, "higher_is_better": True, "vs_baseline": None, "dtype": "bf16x3",
@@ -536,15 +581,26 @@ def main():
         return ms
 
     # ---- arm 1: inputs resident in HBM ---------------------------------------------------------
+    kept_step, kept = [-1], []  # --dump-outputs: (masks, iou) of every request of the last timed step
+
     def step_dev(i):
         for c in range(cps):
-            pp.submit(*devin[(i * cps + c) % n_rot])
+            t = pp.submit(*devin[(i * cps + c) % n_rot])
+            if i == kept_step[0]:  # copied on the lane's stream before the lane's next request overwrites its outputs
+                lane = pp.lanes[t % pp.depth]
+                with torch.cuda.stream(lane.stream):
+                    kept.append((lane.masks.clone(), lane.iou.clone()))
 
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()  # samples clocks / throttle reasons over the warm-up and both timed arms
     timed(step_dev, args.warmup)
+    if args.dump_outputs:
+        kept_step[0] = args.steps - 1
     ms_dev = timed(step_dev, args.steps)
+    kept_step[0] = -1
+    outputs = {"masks": torch.cat([m for m, _ in kept]).cpu(), "iou": torch.cat([i for _, i in kept]).cpu()} if kept else None
+    kept.clear()
 
     # single-stream latency of one cloud (no overlap between clouds), for the record
     n_single = max(3, min(24, args.steps))
@@ -595,12 +651,13 @@ def main():
     # ---- config c3 on the same ranks (the sharded workload: strong scaling, collective inside the timed region) ----
     if not args.no_c3 and args.config == "c2" and os.environ.get("PSAM_PROFILE_STAGE") is None:
         try:
-            c3 = run_c3("c3", args, model, dev, dist, rank, world, barrier)
-            line["c3"] = c3
+            line["c3"] = run_c3("c3", args, model, dev, dist, rank, world, barrier, outputs)
         except Exception as e:  # must never break the headline line
             line["c3"] = {"unavailable": repr(e)[:200]}
             if dist is not None:
                 raise
+    if outputs:  # one budget for the outputs of both arms on every rank
+        write_outputs(args.dump_outputs, outputs, DUMP_BYTES // world, n_points=N, tag=dump_tag)
 
     # ---- roofline of the dominant kernel (rank 0) ---------------------------------------------------
     if rank == 0 and not args.no_roofline and pred.graph is not None:

@@ -1,7 +1,7 @@
 """ORACLE tooling (NOT product code): compile the REFERENCE's own CUDA kernels for sm_100a, from the
-sources where they lie under /root/reference (nothing is copied), into oracle/_ref/ (git-ignored, travels
-to the GPU box).  Used by the GPU tests to pin FPS bit-exactness (incl. the tie-break rule) and the
-nearest-neighbour distance against the real reference kernels.
+reference source tree (nothing is copied), into oracle/_ref/ (git-ignored).  `python -m oracle.make_golden --ref-kernels`
+runs them on a GPU and stores their outputs as tests/golden/ref_kernels.npz, against which the GPU tests pin FPS
+bit-exactness (incl. the tie-break rule) and the nearest-neighbour distance.
 
 Sources compiled: third_party/torkit3d/torkit3d/csrc/cuda/{sample_farthest_points,chamfer_distance}_kernel.cu
 with a 10-line pybind shim (oracle/ref_binding.cpp) - the reference's setup.py is not run.

@@ -10,6 +10,9 @@ TwoWayTransformer, PointCloudSAM.predict_masks) is the reference code itself.
 Run here (needs /root/reference):   python -m oracle.make_golden
 Writes tests/golden/*.npz.  Weights are NOT stored (tens of MB); they are re-created from
 ``oracle.torch_ref.build_model(seed=...)`` and pinned by a checksum stored in the fixture.
+
+``python -m oracle.make_golden --ref-kernels`` writes tests/golden/ref_kernels.npz instead: outputs of the reference's
+CUDA kernels built into oracle/_ref by oracle/build_ref.py, on a GPU.
 """
 from __future__ import annotations
 
@@ -187,6 +190,37 @@ def variant_fixture(ref, out_dir):
         torch.cdist = orig
 
 
+REF_FPS_CASES = [(2, 4096, 128, "grid", 1), (1, 700, 64, "grid", 2), (4, 1024, 512, "ball", 3), (1, 32768, 512, "ball", 4),
+                 (2, 3000, 300, "grid", 5), (1, 50, 50, "grid", 6)]                   # B, N, G, kind, seed
+REF_FPS_STREAMING_CASES = [(200000, 48, "ball"), (200000, 40, "grid"), (524288, 40, "ball"), (524288, 24, "grid")]  # N, G, kind
+REF_FPS_STREAMING_SEED = 13                                                          # B = 1
+REF_NN = dict(N=5000, split=1800, seed=9)  # nearest-neighbour distance from xyz[0, :split] to xyz[0, split:]
+
+
+@torch.no_grad()
+def ref_kernel_fixture(out_dir):
+    """Outputs of the reference's own CUDA kernels (sample_farthest_points_kernel.cu, chamfer_distance_kernel.cu) as
+    oracle/build_ref.py compiles them for sm_100a into oracle/_ref; needs a GPU.  Inputs come from oracle/synth."""
+    from oracle import build_ref
+
+    ref = build_ref.load_ref()
+    if ref is None:
+        raise RuntimeError("oracle/_ref is not built: run `python -m oracle.build_ref` next to the reference sources")
+    d = torch.device("cuda", 0)
+    pack = {}
+    for i, (B, N, G, kind, seed) in enumerate(REF_FPS_CASES):
+        xyz, _ = synth.make_batch(B, N, seed, kind)
+        pack[f"fps{i}"] = ref.sample_farthest_points_cuda(xyz.to(d), G).cpu().numpy()
+    for N, G, kind in REF_FPS_STREAMING_CASES:
+        xyz, _ = synth.make_batch(1, N, REF_FPS_STREAMING_SEED, kind)
+        pack[f"fps_streaming_{N}_{G}_{kind}"] = ref.sample_farthest_points_cuda(xyz.to(d), G).cpu().numpy()
+    xyz, _ = synth.make_batch(1, REF_NN["N"], REF_NN["seed"])
+    a, b = xyz[0, :REF_NN["split"]].to(d), xyz[0, REF_NN["split"]:].to(d)
+    pack["nn_dist"] = ref.chamfer_distance_forward_cuda(a[None], b[None])[0][0].cpu().numpy()
+    np.savez_compressed(os.path.join(out_dir, "ref_kernels.npz"), **pack)
+    print("reference kernel fixture written:", {k: v.shape for k, v in pack.items()})
+
+
 def _sorted_groups(out):
     """Group features with the K members of every group ordered by key index (the reference's topk order is unspecified)."""
     order = torch.argsort(out["knn_idx"], dim=-1)
@@ -196,9 +230,11 @@ def _sorted_groups(out):
 @torch.no_grad()
 def main():
     torch.set_num_threads(8)
-    ref = import_reference()
     out_dir = os.path.join(REPO, "tests", "golden")
     os.makedirs(out_dir, exist_ok=True)
+    if "--ref-kernels" in sys.argv:
+        return ref_kernel_fixture(out_dir)
+    ref = import_reference()
     if "--only-variants" in sys.argv:
         return variant_fixture(ref, out_dir)
     sampler_fixture(ref, out_dir)

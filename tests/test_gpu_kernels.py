@@ -9,6 +9,7 @@ import torch
 pytestmark = pytest.mark.gpu
 
 from oracle import synth, tokenizer_ref, torch_ref  # noqa: E402
+from oracle.make_golden import REF_FPS_CASES, REF_FPS_STREAMING_CASES, REF_FPS_STREAMING_SEED, REF_NN  # noqa: E402
 
 
 def _ops():
@@ -62,41 +63,33 @@ def test_fps_degenerate_and_errors():
         sample_farthest_points(torch.zeros(1, 4, 3), 2)  # CPU tensor: no fallback
 
 
-def test_fps_against_reference_cuda_kernel():
-    """The reference's own kernel compiled for sm_100a (oracle/_ref, built by oracle/build_ref.py)."""
-    from oracle import build_ref
-
-    ref = build_ref.load_ref()
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
+def test_fps_against_reference_cuda_kernel(golden_dir):
+    """Against the outputs of the reference's own kernel compiled for sm_100a (tests/golden/ref_kernels.npz, written by
+    oracle/make_golden.py --ref-kernels)."""
     ops = _ops()
-    for (B, N, G, kind, seed) in [(2, 4096, 128, "grid", 1), (1, 700, 64, "grid", 2), (4, 1024, 512, "ball", 3),
-                                  (1, 32768, 512, "ball", 4), (2, 3000, 300, "grid", 5), (1, 50, 50, "grid", 6)]:
+    z = np.load(os.path.join(golden_dir, "ref_kernels.npz"))
+    for i, (B, N, G, kind, seed) in enumerate(REF_FPS_CASES):
         xyz, _ = synth.make_batch(B, N, seed, kind)
-        x = xyz.to(_dev())
-        want = ref.sample_farthest_points_cuda(x, G).cpu()
-        got, _ = ops.fps(x, G)
+        want = torch.from_numpy(z[f"fps{i}"])
+        got, _ = ops.fps(xyz.to(_dev()), G)
         assert torch.equal(got.cpu(), want), (B, N, G, kind)
         assert (tokenizer_ref.fps(xyz.numpy(), G) == want.numpy()).all(), "oracle vs reference kernel"
 
 
-@pytest.mark.parametrize("N,G,kind", [(200000, 48, "ball"), (200000, 40, "grid"), (524288, 40, "ball"), (524288, 24, "grid")])
-def test_fps_streaming_plan_beyond_cluster_registers(N, G, kind):
+@pytest.mark.parametrize("N,G,kind", REF_FPS_STREAMING_CASES)
+def test_fps_streaming_plan_beyond_cluster_registers(N, G, kind, golden_dir):
     """N > 131072 no longer fits the 16-CTA register plan: the multi-cluster / streaming plan must reproduce the reference
     kernel (sample_farthest_points_kernel.cu:8-104: fmaf chain + bit-reversed tie-break) bit for bit, against the C
-    oracle and - when oracle/_ref travelled - against the reference's own kernel compiled for sm_100a."""
-    from oracle import build_ref
-
+    oracle and against the outputs of the reference's own kernel compiled for sm_100a (tests/golden/ref_kernels.npz)."""
     ops = _ops()
-    xyz, _ = synth.make_batch(1, N, 13, kind)
+    xyz, _ = synth.make_batch(1, N, REF_FPS_STREAMING_SEED, kind)
     x = xyz.to(_dev())
     got, centers = ops.fps(x, G)
     want = tokenizer_ref.fps(xyz.numpy(), G)
     assert np.array_equal(got.cpu().numpy(), want), f"first mismatch at {np.nonzero(got.cpu().numpy() != want)[1][:3]}"
     assert torch.equal(centers.cpu(), torch.gather(xyz, 1, torch.from_numpy(want)[..., None].expand(-1, -1, 3)))
-    ref = build_ref.load_ref()
-    if ref is not None:
-        assert torch.equal(ref.sample_farthest_points_cuda(x, G).cpu(), got.cpu())
+    ref = np.load(os.path.join(golden_dir, "ref_kernels.npz"))[f"fps_streaming_{N}_{G}_{kind}"]
+    assert np.array_equal(ref, got.cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -149,19 +142,16 @@ def test_group_gather_and_interp():
     torch.testing.assert_close(torch.sort(ww.cpu(), -1).values, torch.sort(wwt, -1).values, atol=2e-6, rtol=1e-5)
 
 
-def test_nn_distance_vs_reference_and_bruteforce():
+def test_nn_distance_vs_reference_and_bruteforce(golden_dir):
     ops = _ops()
-    xyz, _ = synth.make_batch(1, 5000, 9)
-    a, b = xyz[0, :1800].to(_dev()), xyz[0, 1800:].to(_dev())
+    xyz, _ = synth.make_batch(1, REF_NN["N"], REF_NN["seed"])
+    a, b = xyz[0, :REF_NN["split"]].to(_dev()), xyz[0, REF_NN["split"]:].to(_dev())
     got = ops.nn_distance(a, b)
     want = (torch.cdist(a.cpu().double(), b.cpu().double()) ** 2).min(dim=1).values.float()
     torch.testing.assert_close(got.cpu(), want, atol=1e-7, rtol=1e-5)
-    from oracle import build_ref
-
-    ref = build_ref.load_ref()
-    if ref is not None:
-        d1 = ref.chamfer_distance_forward_cuda(a[None], b[None])[0][0]
-        torch.testing.assert_close(got, d1, atol=1e-7, rtol=1e-6)
+    # the reference's chamfer kernel compiled for sm_100a (tests/golden/ref_kernels.npz)
+    d1 = torch.from_numpy(np.load(os.path.join(golden_dir, "ref_kernels.npz"))["nn_dist"])
+    torch.testing.assert_close(got.cpu(), d1, atol=1e-7, rtol=1e-6)
 
 
 # ------------------------------------------------------------------------------------------------
