@@ -296,6 +296,37 @@ int psam_add_bcast_f32(const float* a, const float* b, long long n, long long ch
 int psam_split_f32(const float* x, long long ld, long long rows, int D, void* y_hi, long long y_plane,
                    long long ldy_s, long long pitch, cudaStream_t stream);
 
+/* ---- automatic mask generation ----------------------------------------------------------------- */
+/* Candidate masks are bit-packed: bits [R, W] uint32 with W = ceil(N / 32), bit j of word w = point 32 w + j, tail bits 0.
+ * The reference ships no automatic mask generator; the semantics are this project's, following SAM's
+ * SamAutomaticMaskGenerator (segment_anything/automatic_mask_generator.py): see DESIGN.md, "Automatic mask generation". */
+
+/* For R rows of logits [R, N] (one row per candidate) and their predicted IoU iou_pred [R], in one pass:
+ * bits[r] = (logit > mask_threshold), area[r] = popcount, stability[r] = #(logit > t + off) / #(logit > t - off) as an fp32
+ * division of the integer counts (0 when the denominator is 0; SAM's calculate_stability_score), keep[r] = 1 iff
+ * iou_pred > pred_iou_thresh && stability >= stability_thresh && area > 0.  Output pointers may point into a larger
+ * candidate table (the caller offsets them by the chunk's first row). */
+int psam_mask_stats_f32(const float* logits, const float* iou_pred, int R, int N, float mask_threshold, float stability_offset,
+                        float pred_iou_thresh, float stability_thresh, uint32_t* bits, int* area, float* stability,
+                        unsigned char* keep, cudaStream_t stream);
+
+/* Pairwise IoU of two bit-mask sets a [Ka, W], b [Kb, W]: iou [Ka, Kb] = inter / (area_a + area_b - inter) as an fp32
+ * division of exact integer counts (0 when the union is 0); inter [Ka, Kb] int32 may be NULL. */
+int psam_mask_iou_u32(const uint32_t* a_bits, int Ka, const uint32_t* b_bits, int Kb, int W, float* iou, int* inter,
+                      cudaStream_t stream);
+
+/* Greedy mask NMS over K candidates (bits [K, W], area / score / keep [K] from psam_mask_stats_f32):
+ * the candidates with keep != 0, in order of score descending (ties: lower index first), are kept unless an earlier KEPT
+ * candidate has IoU > nms_thresh with them.  keep_idx [K] int32 = kept candidate indices in that order, -1 after the last;
+ * *kept_count (device) = their number.  No host synchronisation: every launch is sized for K.  K <= 16384
+ * (PSAM_ERR_UNSUPPORTED beyond).  workspace: psam_mask_nms_workspace_bytes(K, W) bytes, 16-byte aligned. */
+size_t psam_mask_nms_workspace_bytes(int K, int W);
+int psam_mask_nms(const uint32_t* bits, const int* area, const float* score, const unsigned char* keep, int K, int W,
+                  float nms_thresh, int* keep_idx, int* kept_count, void* workspace, cudaStream_t stream);
+
+/* out [k, N] bytes (0 / 1) = the bits of rows rows[0..k) (rows NULL: rows 0..k-1). */
+int psam_mask_unpack_u8(const uint32_t* bits, int W, const int* rows, int k, int N, unsigned char* out, cudaStream_t stream);
+
 const char* psam_version(void);
 
 #ifdef __cplusplus

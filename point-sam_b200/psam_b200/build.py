@@ -9,7 +9,7 @@ PKG = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(PKG, "csrc")
 LIBDIR = os.path.join(PKG, "lib")
 LIB = os.path.join(LIBDIR, "libpsam_b200.so")
-SOURCES = ["fps.cu", "knn.cu", "gemm_tc.cu", "attention_tc.cu", "elementwise.cu"]
+SOURCES = ["fps.cu", "knn.cu", "gemm_tc.cu", "attention_tc.cu", "elementwise.cu", "masks.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--use_fast_math=false"]
 

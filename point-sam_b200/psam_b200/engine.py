@@ -942,3 +942,57 @@ def _decoder_heads(pk, queries, f0, aux, Z, T, G, D, rep, ids, mask_slice, dev):
     if pk.iou_sigmoid:
         y = torch.sigmoid(y)
     return masks, y[:, mask_slice].contiguous()
+
+
+# ------------------------------------------------------------------------------------------------
+# automatic mask generation (SAM's SamAutomaticMaskGenerator restated for point clouds: DESIGN.md)
+# ------------------------------------------------------------------------------------------------
+AMG_MAX_CANDIDATES = 16384  # psam_mask_nms sorts the candidates in one CTA's shared memory
+
+
+def run_amg_prompts(cloud, P: int) -> torch.Tensor:
+    """The P prompt points [1, P, 3] = the points ops.fps(coords, P) selects.  FPS is prefix-stable, so for P <= G they are
+    the first P centres the encoder's grouper already selected."""
+    patches = cloud["patches"]
+    if "fps_idx" in patches and P <= patches["centers"].shape[1]:
+        return patches["centers"][:, :P]
+    return ops.fps(cloud["coords"], P)[1]
+
+
+def run_automatic_masks(model, cloud, prompts: torch.Tensor, params) -> dict:
+    """Segment everything: every prompt point [1, P, 3] is decoded with multimask output (candidate 3 p + m), each chunk of
+    `points_per_batch` prompts is reduced to bit-packed masks + area / stability / filter flag right after its decode (its
+    fp32 logits do not outlive the chunk), then one NMS over all candidates and ONE host read (kept count and the prompt
+    range flag).  cloud: the dict PointCloudSAM._encode returns (the set_pointcloud cache).  params: a mapping with
+    points_per_batch, pred_iou_thresh, stability_score_thresh, stability_score_offset, mask_threshold, nms_thresh."""
+    coords, patches = cloud["coords"], cloud["patches"]
+    dev = coords.device
+    N, P = coords.shape[1], prompts.shape[1]
+    K = 3 * P
+    W = ops.mask_words(N)
+    table = (torch.empty((K, W), dtype=torch.int32, device=dev), torch.empty(K, dtype=torch.int32, device=dev),
+             torch.empty(K, dtype=torch.float32, device=dev), torch.empty(K, dtype=torch.uint8, device=dev))
+    scores = torch.empty(K, dtype=torch.float32, device=dev)
+    dense = run_mask_encoder(model.mask_encoder, None, coords, patches["centers"], patches["knn_idx"])
+    step = int(params["points_per_batch"])
+    for s in range(0, P, step):
+        pts = prompts[0, s:s + step].unsqueeze(1)  # [Z, 1, 3]: one positive point per prompt
+        Z = pts.shape[0]
+        sparse = run_point_encoder(model.point_encoder, pts, torch.ones((Z, 1), dtype=torch.int32, device=dev), check=False)
+        masks, iou = run_mask_decoder(model.mask_decoder, cloud["pc_embeddings"], cloud["pc_pe"], sparse, dense, cloud["aux"], True)
+        iou = iou.reshape(-1)
+        ops.mask_stats(masks, iou, params["mask_threshold"], params["stability_score_offset"], params["pred_iou_thresh"],
+                       params["stability_score_thresh"], out=table, row0=3 * s)
+        scores[3 * s:3 * (s + Z)].copy_(iou)
+    bits, area, stability, keep = table
+    keep_idx, count = ops.mask_nms(bits, area, scores, keep, params["nms_thresh"])
+    flag = bad_flag(dev)
+    n, bad = torch.cat([count, flag]).tolist()
+    if bad:
+        flag.zero_()
+        raise ValueError("Input coordinates must be normalized to [-1, 1].")
+    rows = keep_idx[:n]
+    idx = rows.long()
+    prompt_index = idx // 3
+    return dict(masks=ops.mask_unpack(bits, N, rows), iou_preds=scores[idx], stability_scores=stability[idx],
+                areas=area[idx].long(), prompt_coords=prompts[0, prompt_index], prompt_index=prompt_index, mask_index=idx % 3)

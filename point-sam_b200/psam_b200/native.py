@@ -62,6 +62,7 @@ EXPORTS = [
     "psam_gemm_bf16x3", "psam_gemm_rowln_bf16x3", "psam_attention_bf16x3", "psam_attention_bf16x3_twopass", "psam_linear_f32", "psam_layernorm_f32", "psam_swiglu_ln", "psam_small_in_linear",
     "psam_group_max", "psam_softmax_split", "psam_transpose_split", "psam_posenc_f32", "psam_attention_f32",
     "psam_decoder_prepare", "psam_interp_ln_gelu", "psam_mask_dot", "psam_add_bcast_f32", "psam_split_f32", "psam_split_add_f32",
+    "psam_mask_stats_f32", "psam_mask_iou_u32", "psam_mask_nms_workspace_bytes", "psam_mask_nms", "psam_mask_unpack_u8",
     "psam_version",
 ]
 
@@ -80,6 +81,8 @@ def lib():
         L.psam_version.restype = ctypes.c_char_p
         L.psam_border_prompt_workspace_bytes.restype = c_size_t
         L.psam_border_prompt_workspace_bytes.argtypes = [i, i, i]
+        L.psam_mask_nms_workspace_bytes.restype = c_size_t
+        L.psam_mask_nms_workspace_bytes.argtypes = [i, i]
         sig = {
             "psam_fps_f32": [p, i, i, i, p, p, p, p],
             "psam_knn_f32": [p, p, i, i, i, i, p, p, p],
@@ -108,6 +111,10 @@ def lib():
             "psam_add_bcast_f32": [p, p, ll, ll, ll, ll, p, p],
             "psam_split_f32": [p, ll, ll, i, p, ll, ll, ll, p],
             "psam_split_add_f32": [p, p, ll, ll, i, p, ll, ll, ll, p],
+            "psam_mask_stats_f32": [p, p, i, i, f, f, f, f, p, p, p, p, p],
+            "psam_mask_iou_u32": [p, i, p, i, i, p, p, p],
+            "psam_mask_nms": [p, p, p, p, i, i, f, p, p, p, p],
+            "psam_mask_unpack_u8": [p, i, p, i, i, p, p],
         }
         for name, args in sig.items():
             fn = getattr(L, name)

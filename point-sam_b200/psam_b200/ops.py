@@ -329,3 +329,73 @@ def split_f32(x: torch.Tensor, out: Split, add: Optional[torch.Tensor] = None):
         nv.check(nv.lib().psam_split_add_f32(nv.ptr(x), nv.ptr(add), x.shape[-1], rows, x.shape[-1], out.ptr(), out.plane, out.pitch,
                                              out.pitch, nv.stream()), "split_add_f32")
 
+
+# ------------------------------------------------------------------------------------------------
+# automatic mask generation: bit-packed candidate masks (bit j of word w = point 32 w + j)
+def mask_words(N: int) -> int:
+    return (N + 31) // 32
+
+
+def mask_stats(logits: torch.Tensor, iou_pred: torch.Tensor, mask_threshold: float, stability_offset: float,
+               pred_iou_thresh: float, stability_thresh: float, out=None, row0: int = 0):
+    """logits [R, N] (any leading shape flattened to rows), iou_pred [R] -> (bits [R, W] int32, area [R] int32,
+    stability [R] fp32, keep [R] uint8).  out = (bits, area, stability, keep) of a larger candidate table: rows
+    row0 .. row0 + R are written (psam_mask_stats_f32)."""
+    N = logits.shape[-1]
+    R = logits.numel() // N
+    if logits.dtype != torch.float32 or iou_pred.dtype != torch.float32 or iou_pred.numel() != R:
+        raise ValueError("mask_stats: fp32 logits [R, N] and fp32 iou_pred [R] expected")
+    if not logits.is_contiguous() or not iou_pred.is_contiguous():
+        raise ValueError("mask_stats: logits and iou_pred must be contiguous")
+    W = mask_words(N)
+    dev = logits.device
+    if out is None:
+        out = (torch.empty((R, W), dtype=torch.int32, device=dev), torch.empty(R, dtype=torch.int32, device=dev),
+               torch.empty(R, dtype=torch.float32, device=dev), torch.empty(R, dtype=torch.uint8, device=dev))
+        row0 = 0
+    bits, area, stab, keep = out
+    if bits.shape[1] != W or row0 < 0 or row0 + R > bits.shape[0] or any(t.shape[0] != bits.shape[0] for t in (area, stab, keep)):
+        raise ValueError("mask_stats: output table too small for rows row0 .. row0 + R")
+    nv.check(nv.lib().psam_mask_stats_f32(nv.ptr(logits), nv.ptr(iou_pred), R, N, float(mask_threshold), float(stability_offset),
+                                          float(pred_iou_thresh), float(stability_thresh), nv.ptr(bits) + 4 * W * row0,
+                                          nv.ptr(area) + 4 * row0, nv.ptr(stab) + 4 * row0, nv.ptr(keep) + row0, nv.stream()),
+             "mask_stats_f32")
+    return out
+
+
+def mask_iou(a_bits: torch.Tensor, b_bits: torch.Tensor, want_inter: bool = False):
+    """IoU [Ka, Kb] fp32 (and the int32 intersections) of two bit-mask sets [Ka, W], [Kb, W] (psam_mask_iou_u32)."""
+    if a_bits.dtype != torch.int32 or b_bits.dtype != torch.int32 or a_bits.shape[1] != b_bits.shape[1]:
+        raise ValueError("mask_iou: int32 bit masks with the same number of words expected")
+    a, b = a_bits.contiguous(), b_bits.contiguous()
+    Ka, W = a.shape
+    Kb = b.shape[0]
+    iou = torch.empty((Ka, Kb), dtype=torch.float32, device=a.device)
+    inter = torch.empty((Ka, Kb), dtype=torch.int32, device=a.device) if want_inter else None
+    nv.check(nv.lib().psam_mask_iou_u32(nv.ptr(a), Ka, nv.ptr(b), Kb, W, nv.ptr(iou), nv.ptr(inter), nv.stream()), "mask_iou_u32")
+    return (iou, inter) if want_inter else iou
+
+
+def mask_nms(bits: torch.Tensor, area: torch.Tensor, score: torch.Tensor, keep: torch.Tensor, nms_thresh: float):
+    """Greedy NMS of the candidates with keep != 0 (psam_mask_nms): keep_idx [K] int32 (kept candidates in score order,
+    -1 after the last) and kept_count [1] int32, both on the device (nothing is read back)."""
+    K, W = bits.shape
+    if bits.dtype != torch.int32 or area.dtype != torch.int32 or score.dtype != torch.float32 or keep.dtype != torch.uint8:
+        raise ValueError("mask_nms: int32 bits / areas, fp32 scores and uint8 keep flags expected")
+    dev = bits.device
+    keep_idx = torch.empty(K, dtype=torch.int32, device=dev)
+    count = torch.empty(1, dtype=torch.int32, device=dev)
+    ws = torch.empty(nv.lib().psam_mask_nms_workspace_bytes(K, W), dtype=torch.uint8, device=dev)
+    nv.check(nv.lib().psam_mask_nms(nv.ptr(bits), nv.ptr(area), nv.ptr(score), nv.ptr(keep), K, W, float(nms_thresh),
+                                    nv.ptr(keep_idx), nv.ptr(count), nv.ptr(ws), nv.stream()), "mask_nms")
+    return keep_idx, count
+
+
+def mask_unpack(bits: torch.Tensor, N: int, rows: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """bool [k, N] masks of the bit rows `rows` (int32 [k]; None: all rows) (psam_mask_unpack_u8)."""
+    r = rows.to(torch.int32).contiguous() if rows is not None else None
+    k = r.numel() if r is not None else bits.shape[0]
+    out = torch.empty((k, N), dtype=torch.uint8, device=bits.device)
+    if k:
+        nv.check(nv.lib().psam_mask_unpack_u8(nv.ptr(bits), bits.shape[1], nv.ptr(r), k, N, nv.ptr(out), nv.stream()), "mask_unpack_u8")
+    return out.view(torch.bool)
